@@ -12,6 +12,7 @@ decommitments and the postcard proof bytes.  Host-side trace FILLING is outside 
     python bench.py --impl reference ...                     # CPU arm: the oracle's whole proof of the SAME machine, really executed (2^18-row sample; --ref-log-rows 20 = full size)
     python bench.py --fft-sweep [--gpus N]                   # BASELINE configs[4]: Circle-FFT M31 elems/s, 2^16..2^26
     python bench.py --log-rows 22 --steps 2 --warmup 1       # BASELINE configs[2]: a 2^22-row full proof on one GPU
+    python bench.py --dump-outputs DIR ...                   # also writes the last timed proof's outputs as DIR/*.npy (compare two builds)
 
   value   cycles/s with the filled trace (trees 0+1 evaluations) already RESIDENT in HBM when the timed region starts;
   e2e     the same proof through the public host-column API: pinned HOST trace columns in (packed: byte-valued columns travel as
@@ -71,7 +72,15 @@ def parse():
     ap.add_argument("--fft-sweep", action="store_true")
     ap.add_argument("--sweep-logs", default="16,18,20,22,24,26")
     ap.add_argument("--sweep-mib", type=int, default=1024, help="MiB of evaluations per sweep point and GPU")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed proof returned (rank 0's) as DIR/<name>.npy in float64: proof bytes, "
+                         "claimed LogUp sums, the three tree roots, the lookup parameters; inputs are seeded, so two builds can be compared file by file")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.fft_sweep:
+        ap.error("--dump-outputs writes a proof's outputs; --fft-sweep computes none")
+    return args
 
 
 class ClockSampler:
@@ -198,12 +207,12 @@ def fill_trace(m, seed):
 
 
 def oracle_full_prove(m, cols, mult):
-    """One whole proof by the oracle (CPU restatement of the same pipeline), all host threads; returns (seconds, proof, aux)."""
+    """One whole proof by the oracle (CPU restatement of the same pipeline), all host threads; returns (seconds, proof, claimed, aux)."""
     from nexus_zkvm_b200 import machine as M
     from tests.oracle_backend import OracleBackend
     t0 = time.perf_counter()
     proof, claimed, aux = M.prove(m, OracleBackend(), cols, mult, config=CONFIG)
-    return time.perf_counter() - t0, proof, aux
+    return time.perf_counter() - t0, proof, claimed, aux
 
 
 def run_reference(args):
@@ -220,7 +229,9 @@ def run_reference(args):
     ref_rows = min(args.ref_log_rows, args.log_rows)
     m = make_machine(args, ref_rows)
     cols, mult = fill_trace(m, 0)
-    t, proof, _aux = oracle_full_prove(m, cols, mult)   # ONE step: a CPU proof of this size takes minutes
+    t, proof, claimed, aux = oracle_full_prove(m, cols, mult)   # ONE step: a CPU proof of this size takes minutes
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, proof, claimed, aux)
     value = (1 << ref_rows) / t
     line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": 1, "warmup": 0,
             "ms_per_step": t * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u32 (M31)",
@@ -231,6 +242,18 @@ def run_reference(args):
             "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0, "reference_log_rows": ref_rows, "note": "steps/warmup fixed to 1/0: one CPU proof takes minutes"}
     print(json.dumps(line), flush=True)
+
+
+def dump_outputs(d, proof, claimed, aux):
+    """What a caller of machine.prove receives, as float64 arrays (every value is a byte or an M31 element < 2^31: exact in float64)."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    out = {"proof": np.frombuffer(proof, dtype=np.uint8),
+           "claimed_sums": np.array(claimed, dtype=np.uint32).reshape(-1, 4),
+           "roots": np.frombuffer(b"".join(aux["roots"]), dtype=np.uint8).reshape(-1, 32),
+           "params": np.array(aux["params"], dtype=np.uint32).reshape(-1, 4)}
+    for name, a in out.items():
+        np.save(os.path.join(d, name + ".npy"), a.astype(np.float64))
 
 
 def load_peaks():
@@ -358,6 +381,8 @@ def main():
         ms_per_step = float(ms.item()) / args.steps
         launches = (ctx.launches - l0) * world
         value = world * n_rows / (ms_per_step * 1e-3)
+        if rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, last["proof"], last["claimed"], last["aux"])
 
         # ---- e2e: pinned host columns -> proof bytes on the host, copies inside the timed region
         e2e = None
@@ -409,7 +434,7 @@ def main():
             orc.set_num_threads(os.cpu_count() or 1)
             ms_ = make_machine(args, args.cpu_sample_log_rows)
             cs, mu = fill_trace(ms_, 0)
-            tcpu, _p, _a = oracle_full_prove(ms_, cs, mu)
+            tcpu, _p, _c, _a = oracle_full_prove(ms_, cs, mu)
             cpu_baseline = {"value": (1 << args.cpu_sample_log_rows) / tcpu, "unit": UNIT, "cores": orc.num_threads(), "kind": "port",
                             "sample": f"one whole proof of the same machine at 2^{args.cpu_sample_log_rows} rows ({tcpu:.1f} s); `--impl reference` runs a 2^{min(args.ref_log_rows, args.log_rows)}-row proof"}
         except Exception as e:  # the GPU numbers must still be reported
